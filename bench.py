@@ -6,6 +6,7 @@ reference's CPU path (oracle port) beside it.
     python bench.py --workload hashbucket ...                      # configs[4]: HashBucket 40 x int64
     python bench.py --workload movielens ...                       # configs[3]: JoinGroupby + TargetEncoding
     python bench.py --impl reference [--workload ...] ...          # the reference's CPU path, all host cores
+    python bench.py ... --dump-outputs DIR                         # + the last timed step's outputs, sampled
 
 Default workload (criteo): a "step" = Workflow.fit(dataset) + Workflow.transform(dataset) over the
 whole HBM-resident table of 2.5e8 rows per GPU (SURVEY.md 8d C2), categorical cardinalities of the
@@ -22,6 +23,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -239,17 +241,82 @@ def make_table(workload, rows, device, rank, profile_rows):
     return synth.movielens_frame(rows, device=device, rank=rank)
 
 
-def run_step(nvt, wf, parts, fit=True):
+def run_step(nvt, wf, parts, fit=True, sink=None):
     """one pass of the hot path over the resident table: fit (accumulated over the partitions,
     artefact files written — Workflow.fit joins its writer threads), then transform partition
-    by partition (the outputs of one partition live at a time)"""
+    by partition (the outputs of one partition live at a time; `sink(i, part)` sees each)"""
     ds = nvt.Dataset(list(parts))
     if fit:
         wf.fit(ds)
     out = None
-    for part in wf.transform(ds).partitions():
+    for i, part in enumerate(wf.transform(ds).partitions()):
+        if sink is not None:
+            sink(i, part)
         out = part
     return out
+
+
+DUMP_BYTES = 64 << 20        # --dump-outputs writes at most this much
+DUMP_ROWS = 1 << 17
+
+
+class OutputSample:
+    """--dump-outputs: the same seeded sample of rows of every output column of one step.
+    take(i, part) gathers the sampled rows of output partition i on the device while the step
+    runs (a step keeps one partition's outputs alive at a time); save(dir) writes <column>.npy
+    and row_index.npy (the sampled rows of the table).  Float32 columns stay float32, all other
+    columns become float64 (integers below 2^53 exactly), nulls become NaN."""
+
+    def __init__(self, part_rows, ncols, device, seed=0):
+        import numpy as np
+        import torch
+        total = sum(part_rows)
+        n = min(total, DUMP_ROWS, DUMP_BYTES // (8 * (ncols + 1)))
+        self.rows = np.sort(np.random.default_rng(seed).choice(total, size=n, replace=False))
+        self.part_rows = list(part_rows)
+        bounds = np.cumsum([0] + self.part_rows)
+        self.local = [torch.from_numpy(self.rows[(self.rows >= s) & (self.rows < e)] - s).to(device)
+                      for s, e in zip(bounds[:-1], bounds[1:])]
+        self.parts = [None] * len(self.part_rows)
+
+    def take(self, i, part):
+        import torch
+        if len(part) != self.part_rows[i]:
+            raise ValueError(f"output partition {i} has {len(part)} rows, its input {self.part_rows[i]}")
+        idx, got = self.local[i], {}
+        for name, col in part.items():
+            if col.offsets is not None:
+                raise ValueError(f"--dump-outputs: list column {name} is not supported")
+            valid = None
+            if col.validity is not None:      # Arrow bitmask: bit (r & 7) of byte (r >> 3)
+                valid = (col.validity.index_select(0, idx >> 3) >> (idx & 7).to(torch.uint8)) & 1
+            got[name] = (col.data.index_select(0, idx), valid)
+        self.parts[i] = got
+
+    def save(self, out_dir):
+        import numpy as np
+        import torch
+        if any(p is None for p in self.parts):
+            raise RuntimeError("--dump-outputs: the timed step did not produce every partition")
+        arrays = {"row_index": self.rows.astype(np.float64)}
+        for name in self.parts[0]:
+            if name in arrays:
+                raise ValueError(f"--dump-outputs: output column {name} clashes with row_index.npy")
+            vals = torch.cat([p[name][0] for p in self.parts]).cpu().numpy()
+            if vals.dtype.kind in "iu" and vals.size and np.abs(vals.astype(np.float64)).max() >= 2.0 ** 53:
+                raise ValueError(f"--dump-outputs: integer column {name} is not exact in float64")
+            out = vals.astype(np.float32 if vals.dtype == np.float32 else np.float64)
+            valid = [np.ones(len(d), bool) if v is None else v.cpu().numpy() == 1
+                     for d, v in (p[name] for p in self.parts)]
+            out[~np.concatenate(valid)] = np.nan
+            arrays[name] = out
+        total = sum(a.nbytes for a in arrays.values())
+        if total > DUMP_BYTES:
+            raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte limit")
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+        return sorted(arrays), total
 
 
 def host_partitions(frame, nparts):
@@ -397,7 +464,7 @@ def _same_state(a, b):
     return True
 
 
-def parity_gate(nvt, workload, rank, world, dev):
+def parity_gate(nvt, workload, rank, world, dev, tmp_root):
     """A small seeded table (every rank a different shard) through the SAME code paths the timed
     run takes (NVTB_RUNS_MIN_KEYS lowered so that the sorted accumulator is exercised):
       1. the fitted state (vocabulary keys / sizes / null counts, means / stds, group tables) of
@@ -473,7 +540,7 @@ def parity_gate(nvt, workload, rank, world, dev):
                                                 for c in df.columns if c not in exact]
             return out
 
-        tmp = f"/tmp/nvtb_gate_rank{rank}"
+        tmp = os.path.join(tmp_root, "gate")
         wf = build_workflow(nvt, workload, tmp)
         ds = nvt.Dataset(cut(local, 3))
         if workload != "hashbucket":
@@ -581,7 +648,14 @@ def main():
                     help="NVTB_ARTIFACTS for the timed steps (eager = library default)")
     ap.add_argument("--sweep", default="", help="hashbucket: comma-separated row counts for the roofline curve")
     ap.add_argument("--pyprofile", action="store_true", help="cProfile one extra step to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one computed (rank 0): every output "
+                         f"column at the same {DUMP_ROWS} seeded sample rows, as DIR/<column>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     os.environ["NVTB_ARTIFACTS"] = args.artifacts
     args.warmup = max(args.warmup, 0)
     wl = args.workload
@@ -636,14 +710,17 @@ def main():
             dist.barrier()
             torch.cuda.synchronize()
 
+    # the artefact files of the fits go to a private directory, removed at exit: the source tree
+    # may be read-only, and a fixed /tmp name may belong to another user of the machine
+    tmp_root = tempfile.TemporaryDirectory(prefix=f"nvtb_bench_rank{rank}_", ignore_cleanup_errors=True)
     gate = {"status": "skipped"}
     if not args.no_gate:
-        gate = parity_gate(nvt, wl, rank, world, dev)
+        gate = parity_gate(nvt, wl, rank, world, dev, tmp_root.name)
         torch.cuda.empty_cache()
 
     table = make_table(wl, rows, dev, rank, args.profile_rows)
     frame = cut(table, args.parts)
-    out_dir = f"/tmp/nvtb_bench_rank{rank}"
+    out_dir = os.path.join(tmp_root.name, "bench")
     wf = build_workflow(nvt, wl, out_dir, args.int32_outputs)
     has_fit = wl != "hashbucket"
 
@@ -672,7 +749,7 @@ def main():
         pr.disable()
         pstats.Stats(pr, stream=sys.stderr).sort_stats("cumulative").print_stats(35)
 
-    def timed(parts, steps, warmup, with_profile=True, sampler=None):
+    def timed(parts, steps, warmup, with_profile=True, sampler=None, sink=None):
         for _ in range(warmup):
             out = run_step(nvt, wf, parts, has_fit)
             del out
@@ -682,8 +759,8 @@ def main():
         launches0 = engine.kernel_launches
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
-        for _ in range(steps):
-            out = run_step(nvt, wf, parts, has_fit)
+        for i in range(steps):
+            out = run_step(nvt, wf, parts, has_fit, sink if i == steps - 1 else None)
             del out
         ev1.record()
         sync_all()
@@ -705,8 +782,17 @@ def main():
         del out
     if rank == 0 and time.time() - t_sampler < 1.5:      # nvidia-smi start-up must be over
         time.sleep(1.5 - (time.time() - t_sampler))
-    ms_per_step, launches, prof, clocks = timed(frame, args.steps, max(0, args.warmup - 1), True, sampler)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = OutputSample([len(p) for p in frame], len(wf.output_node.output_columns.names), dev)
+    ms_per_step, launches, prof, clocks = timed(frame, args.steps, max(0, args.warmup - 1), True, sampler,
+                                                dump.take if dump else None)
     value = total_rows / (ms_per_step / 1e3)
+    if dump:
+        names, nbytes = dump.save(args.dump_outputs)
+        sys.stderr.write(f"[bench] last timed step: {len(dump.rows)} sampled rows of {len(names) - 1} output "
+                         f"columns ({nbytes} bytes) written to {args.dump_outputs}\n")
+        dump = None
 
     # per-kernel-family device time (CUDA events on the launching stream)
     fam = {}

@@ -4,6 +4,7 @@ single-process fit over the concatenation of all shards, and the transform of th
 shard must equal the single-process transform of those rows."""
 import os
 import sys
+import tempfile
 
 import torch
 import torch.distributed as dist
@@ -35,14 +36,16 @@ def main():
         return nvt.Workflow((cats >> nvt.ops.Categorify(out_path=path, freq_threshold=2))
                             + (conts >> nvt.ops.FillMissing() >> nvt.ops.Normalize()))
 
+    tmp = tempfile.TemporaryDirectory(prefix=f"nvtb_dist_rank{rank}_")
+
     # distributed fit on the local shard
-    wf = workflow(f"/tmp/nvtb_dist_{rank}")
+    wf = workflow(os.path.join(tmp.name, "dist"))
     wf.fit(nvt.Dataset(mine))
     out = next(iter(wf.transform(nvt.Dataset(mine)).partitions()))
 
     # reference: the same engine, single process, all shards as partitions (no collectives)
     os.environ["NVTB_DISABLE_DIST"] = "1"
-    ref = workflow(f"/tmp/nvtb_dist_ref_{rank}")
+    ref = workflow(os.path.join(tmp.name, "single"))
     ref.fit(nvt.Dataset(shards))
     ref_out = ref.transform(mine)
     os.environ.pop("NVTB_DISABLE_DIST")

@@ -4,6 +4,7 @@ and the rule that the product never touches the oracle or a CPU fallback."""
 import ctypes
 import os
 import re
+import shutil
 import subprocess
 import sys
 
@@ -29,8 +30,10 @@ def test_library_exports_every_header_symbol():
 
 
 def test_library_targets_sm100a_with_256bit_accesses():
-    from nvtabular_b200 import _lib
-    sass = subprocess.run(["cuobjdump", "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    from nvtabular_b200 import _build, _lib
+    # the CUDA toolkit that built the library, also when its bin directory is not on PATH
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.path.dirname(_build._nvcc()), "cuobjdump")
+    sass = subprocess.run([cuobjdump, "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in sass or "SM100a" in sass.upper() or "sm_100" in sass
     assert re.search(r"LDG\.E[.\w]*\.256", sass) and re.search(r"STG\.E[.\w]*\.256", sass)
 
@@ -435,3 +438,66 @@ def test_bench_e2e_rows_fit_the_host_memory_limit():
     assert bench.e2e_rows_within_host_memory(want, bpr, 8, 1 * G) == 1 << 23
     b = bench._host_memory_budget()
     assert b is None or b > 0
+
+
+def test_bench_output_sample_gathers_the_same_rows_of_every_partition(tmp_path):
+    """bench.py --dump-outputs: one seeded sample of rows across uneven partitions, integers as exact
+    float64, float32 kept, nulls of a bitmask column as NaN, the same rows from run to run"""
+    import bench
+    from nvtabular_b200.column import Column, DeviceFrame, pack_validity
+    rng = np.random.default_rng(1)
+    n = 300_007
+    full = {"a": rng.integers(0, 1 << 40, n), "x": rng.standard_normal(n).astype(np.float32),
+            "i": rng.integers(-5, 5, n).astype(np.int32)}
+    valid = rng.random(n) < 0.7
+    frame = DeviceFrame({"a": Column(torch.from_numpy(full["a"])), "x": Column(torch.from_numpy(full["x"])),
+                         "i": Column(torch.from_numpy(full["i"]), pack_validity(torch.from_numpy(valid)))})
+    parts = bench.cut(frame, 3)
+    sample = bench.OutputSample([len(p) for p in parts], 3, "cpu")
+    for i, p in enumerate(parts):
+        sample.take(i, p)
+    names, nbytes = sample.save(str(tmp_path))
+    assert names == ["a", "i", "row_index", "x"] and nbytes <= bench.DUMP_BYTES
+    row = np.load(tmp_path / "row_index.npy")
+    assert row.dtype == np.float64 and len(row) == bench.DUMP_ROWS and (np.diff(row) > 0).all()
+    row = row.astype(np.int64)
+    np.testing.assert_array_equal(row, bench.OutputSample([len(p) for p in parts], 3, "cpu").rows)
+    a, x, i = (np.load(tmp_path / f"{c}.npy") for c in ("a", "x", "i"))
+    assert a.dtype == np.float64 and x.dtype == np.float32 and i.dtype == np.float64
+    np.testing.assert_array_equal(a, full["a"][row].astype(np.float64))
+    np.testing.assert_array_equal(x, full["x"][row])
+    np.testing.assert_array_equal(i, np.where(valid[row], full["i"][row], np.nan))
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs writes every output column of its timed step at the seeded sample
+    rows; a fit + transform of the same table in this process gives the same values"""
+    import json
+    import bench
+    import nvtabular_b200 as nvt
+    rows, parts, profile = 1 << 20, 3, 40_000_000
+    dump = tmp_path / "dump"
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--rows", str(rows), "--parts", str(parts),
+           "--profile-rows", str(profile), "--steps", "2", "--warmup", "1", "--no-e2e", "--no-cpu-baseline",
+           "--no-gate", "--dump-outputs", str(dump)]
+    r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=str(tmp_path))
+    assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-1500:]
+    lines = [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == 2
+    wf = bench.build_workflow(nvt, "criteo", str(tmp_path / "wf"))
+    names = wf.output_node.output_columns.names
+    assert sorted(os.listdir(dump)) == sorted(n + ".npy" for n in names + ["row_index"])
+    assert sum(os.path.getsize(dump / f) for f in os.listdir(dump)) <= bench.DUMP_BYTES
+    row = np.load(dump / "row_index.npy").astype(np.int64)
+    table = bench.make_table("criteo", rows, torch.device("cuda"), 0, profile)
+    wf.fit(nvt.Dataset(bench.cut(table, parts)))
+    out = wf.transform(table)
+    for c in names:
+        got = np.load(dump / f"{c}.npy")
+        exp = out[c].data[torch.from_numpy(row).cuda()].cpu().numpy()
+        assert len(got) == len(row) and not np.isnan(got).any(), c
+        if exp.dtype.kind in "iu":
+            np.testing.assert_array_equal(got, exp.astype(np.float64), err_msg=c)
+        else:
+            np.testing.assert_allclose(got, exp, rtol=1e-9, atol=1e-12, err_msg=c)
