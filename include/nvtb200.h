@@ -394,6 +394,70 @@ int nvtb_comm_allgather(nvtb_comm_t* c, const void* send_dev, void* recv_dev, in
 int nvtb_comm_alltoallv(nvtb_comm_t* c, const void* send_dev, const int64_t* send_counts_host,
                         void* recv_dev, const int64_t* recv_counts_host, int elem_bytes, void* stream);
 
+/* ---- session ops: Groupby, ListSlice, Dataset.shuffle_by_keys (csrc/groupby.cu) ----------
+ * Replace cuDF sort_values + groupby(sort=True, dropna=True).agg + list.get of reference
+ * nvtabular/ops/groupby.py:114-150, 213-240, 290-319, and the numba kernels _calculate_row_sizes
+ * / _slice_rows of nvtabular/ops/list_slice.py:180-228.  A partition is ordered once
+ * (nvtb_sort_rows), cut into groups once (nvtb_segments: the ONE host synchronisation per
+ * Groupby per partition that sizes the outputs, besides the key-range read of the sort), and
+ * every output column is one more pass over that order. */
+
+/* Stable lexicographic row order over nkeys (<= 8) key columns, keys[0] most significant
+ * (reference groupby.py:116 sort_values + :236 groupby(sort=True)).  descending[k] != 0 orders
+ * key k descending (NULL: all ascending).  Rows with a null in any of the first n_drop_null keys
+ * are dropped (dropna=True): they go after the *n_kept_dev kept rows of perm_out.  The other keys
+ * order their nulls last in either direction (na_position="last").  Floating -0.0 equals +0.0.
+ * perm_out: int32[n] row numbers, n < 2^31.  Synchronises once (the keys' value ranges, which
+ * trim the radix passes to the bits in use). */
+int nvtb_sort_rows(const nvtb_col_t* keys_host, const int* descending_host, int nkeys, int n_drop_null,
+                   int64_t n, int32_t* perm_out, int64_t* n_kept_dev, void* stream);
+/* group boundaries of the first *n_kept_dev rows of perm (keys equal <=> same group):
+ * offsets_out[0..n_groups] (int64, room for n_max + 1), offsets_out[n_groups] = n_kept.
+ * Synchronises: the group count and the kept-row count come back to the host. */
+int nvtb_segments(const nvtb_col_t* keys_host, int nkeys, const int32_t* perm, int64_t n_max,
+                  const int64_t* n_kept_dev, int64_t* offsets_out, int64_t* n_groups_host,
+                  int64_t* n_kept_host, void* stream);
+/* out[i] = src[perm[idx[i] + idx_shift]] (idx NULL: perm[i]; perm NULL: no permutation) for
+ * i < n, any 1/4/8-byte dtype; validity_out (4-byte aligned, padded to a multiple of 4 bytes)
+ * is required when src has a validity mask.  The group keys (idx = offsets) and "list"
+ * (the whole permutation) of Groupby. */
+int nvtb_gather_rows(const nvtb_col_t* src_host, const int32_t* perm, const int64_t* idx,
+                     int idx_shift, int64_t n, void* out, uint8_t* validity_out, void* stream);
+/* Scalar aggregations of every group of a value column (reference groupby.py:213-240, pandas
+ * semantics; accumulated in double).  out_host / validity_out_host: 9 slots in the order
+ * count, sum, mean, min, max, std, var, first, last; NULL = not requested.  Output dtypes:
+ * count int32; sum, mean, std, var float32; min, max, first, last the value dtype.  count and
+ * sum (0 when no value) have no validity; mean, min, max (null without a non-null value), std,
+ * var (ddof 1, null below 2 values) need one; first / last (the group's first / last row, a
+ * null stays null) need one when the column has nulls.  Groups of up to 32 rows are reduced by
+ * one thread, longer ones in chunks of 2048 rows, one CTA each, merged with atomics. */
+int nvtb_segment_agg(const nvtb_col_t* val_host, const int32_t* perm, const int64_t* offsets,
+                     int64_t n_groups, void* const* out_host, uint8_t* const* validity_out_host,
+                     void* stream);
+/* median (float32, mean of the two middle values, null without values) and nunique (int32,
+ * distinct non-null values) of groups whose rows are in value order with nulls last: perm from
+ * nvtb_sort_rows over (group keys..., value), offsets from nvtb_segments of the group keys.
+ * n_rows = kept rows.  Either output may be NULL. */
+int nvtb_segment_sorted_agg(const nvtb_col_t* val_host, const int32_t* perm, const int64_t* offsets,
+                            int64_t n_groups, int64_t n_rows, float* median_out,
+                            uint8_t* median_validity_out, int32_t* nunique_out, void* stream);
+/* ListSlice (reference list_slice.py:58-75, 104-142): output row r is the Python slice
+ * row[start:end] of source row s(r) = perm[idx[r] + idx_shift] (NULL perm / idx as in
+ * nvtb_gather_rows), padded at the end to max_elements when pad != 0.  Also the list-row gather
+ * of first / last on list columns (start 0, end INT64_MAX).  Step 1 writes offsets_out[n_rows+1]
+ * and the leaf count; it synchronises unless pad != 0 (offsets r * max_elements).  Step 2 copies
+ * the leaves (pad_value cast to the leaf dtype); validity_out is required when the leaves have
+ * nulls and pads are valid. */
+int nvtb_list_slice_offsets(const int64_t* offsets, int64_t n_rows, const int32_t* perm,
+                            const int64_t* idx, int idx_shift, int64_t start, int64_t end, int pad,
+                            int64_t max_elements, int64_t* offsets_out, int64_t* total_host,
+                            void* stream);
+int nvtb_list_slice(const int64_t* offsets, const nvtb_col_t* leaves_host, int64_t n_rows,
+                    const int32_t* perm, const int64_t* idx, int idx_shift, int64_t start,
+                    int64_t end, int pad, int64_t max_elements, double pad_value,
+                    const int64_t* offsets_out, int64_t total, void* leaves_out,
+                    uint8_t* validity_out, void* stream);
+
 /* ---- inference-time transforms on HOST arrays --------------------------------------------
  * The twin of the reference's pybind11 module nvtabular_cpp.inference
  * (cpp/nvtabular/inference/categorify.cc:31-347, fill.cc:32-124; bound at

@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libnvtb200.so")
-SOURCES = ["scan_kernels.cu", "hashagg.cu", "vocab.cu", "infer.cu", "comm.cu"]
+SOURCES = ["scan_kernels.cu", "hashagg.cu", "vocab.cu", "infer.cu", "comm.cu", "groupby.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",

@@ -94,6 +94,13 @@ _SIGNATURES = {
     "nvtb_groupstats_create": (c_int, [POINTER(c_void_p), c_void_p, c_int64, c_void_p, c_int, c_int64, c_void_p]),
     "nvtb_groupstats_destroy": (c_int, [c_void_p]),
     "nvtb_groupstats_gather": (c_int, [c_void_p, POINTER(nvtb_col_t), c_int64, POINTER(c_int), c_int, POINTER(c_double), POINTER(c_void_p), POINTER(c_int), c_void_p]),
+    "nvtb_sort_rows": (c_int, [POINTER(nvtb_col_t), POINTER(c_int), c_int, c_int, c_int64, c_void_p, c_void_p, c_void_p]),
+    "nvtb_segments": (c_int, [POINTER(nvtb_col_t), c_int, c_void_p, c_int64, c_void_p, c_void_p, POINTER(c_int64), POINTER(c_int64), c_void_p]),
+    "nvtb_gather_rows": (c_int, [POINTER(nvtb_col_t), c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p]),
+    "nvtb_segment_agg": (c_int, [POINTER(nvtb_col_t), c_void_p, c_void_p, c_int64, POINTER(c_void_p), POINTER(c_void_p), c_void_p]),
+    "nvtb_segment_sorted_agg": (c_int, [POINTER(nvtb_col_t), c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "nvtb_list_slice_offsets": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int64, c_int64, c_int, c_int64, c_void_p, POINTER(c_int64), c_void_p]),
+    "nvtb_list_slice": (c_int, [c_void_p, POINTER(nvtb_col_t), c_int64, c_void_p, c_void_p, c_int, c_int64, c_int64, c_int, c_int64, c_double, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -322,6 +322,41 @@ class Dataset:
         self.cpu = True
         return self
 
+    def shuffle_by_keys(self, keys, npartitions: Optional[int] = None) -> "Dataset":
+        """A Dataset whose partitions each hold every row of the key tuples they contain: what
+        Groupby needs (its transform never moves rows between partitions, reference
+        nvtabular/ops/groupby.py:30-35; merlin.io.Dataset.shuffle_by_keys).  Row r goes to
+        partition hash(keys of r) % npartitions (default: the current count), with the value hash
+        of HashBucket; inside a partition rows keep their order (input partition, then row), so ties
+        in Groupby's sort columns resolve as on one partition.  Within one process only."""
+        from .dist import world
+        from .ops.fill import materialize
+        from . import engine
+        if world()[0] > 1:
+            raise NotImplementedError("shuffle_by_keys moves rows within one process only; under "
+                                      "torch.distributed each rank's files must already hold whole key groups")
+        keys = [keys] if isinstance(keys, str) else list(keys)
+        parts = [DeviceFrame({k: materialize(c) for k, c in p.items()}) for p in self.partitions()]
+        k = int(npartitions or len(parts) or 1)
+        whole = _concat_frames(parts)
+        if not len(whole):
+            return Dataset([whole], device=self._device)
+        dest = engine.hash_bucket([whole[c] for c in keys], k)
+        perm, _ = engine.sort_rows([Column(dest)])
+        counts = torch.bincount(dest.long(), minlength=k).tolist()
+        out, start = [], 0
+        for c in counts:
+            p = perm[start:start + c]
+            start += c
+            cols = {}
+            for name, col in whole.items():
+                if col.is_list:
+                    cols[name] = engine.list_slice(col, 0, np.iinfo(np.int64).max, perm=p, n_rows=c)
+                else:
+                    cols[name] = engine.gather_rows(col, p, c)
+            out.append(DeviceFrame(cols))
+        return Dataset(out, device=self._device)
+
     def to_parquet(self, output_path, shuffle=None, out_files_per_proc=None, seed=None, **kwargs):
         """Write the (lazily transformed) dataset as parquet part files — merlin.io.Dataset.to_parquet
         as the reference's benchmark calls it (bench/examples/dask-nvtabular-criteo-benchmark.py:225-237;
@@ -379,6 +414,44 @@ class Dataset:
             tab = tab.take(pa.array(rng.permutation(len(tab))))
             pq.write_table(tab, os.path.join(output_path, f"{prefix}{f}.parquet"))
         return output_path
+
+
+def _concat_columns(cols: List[Column]) -> Column:
+    """rows of several columns one after the other; string dictionaries are merged (codes stay
+    order-preserving) and list offsets rebased"""
+    from .column import pack_validity, unpack_validity
+    if len(cols) == 1:
+        return cols[0]
+    dictionary = None
+    datas = [c.data for c in cols]
+    if any(c.dictionary is not None for c in cols):
+        dictionary = np.array(sorted(set().union(*[set(c.dictionary.tolist()) for c in cols
+                                                   if c.dictionary is not None])), dtype=object)
+        datas = []
+        for c in cols:
+            if c.dictionary is None or not len(c.dictionary):
+                datas.append(torch.zeros_like(c.data))
+                continue
+            lut = torch.from_numpy(np.searchsorted(dictionary, c.dictionary).astype(np.int32)).to(c.data.device)
+            datas.append(lut[c.data.long()])
+    validity = None
+    if any(c.validity is not None for c in cols):
+        validity = pack_validity(torch.cat([unpack_validity(c.validity, c.data.numel(), c.data.device) for c in cols]))
+    offsets = None
+    if cols[0].offsets is not None:
+        pieces, base = [], 0
+        for c in cols:
+            pieces.append(c.offsets[:-1] + base)
+            base += int(c.data.numel())
+        pieces.append(torch.tensor([base], dtype=torch.int64, device=cols[0].data.device))
+        offsets = torch.cat(pieces)
+    return Column(torch.cat(datas), validity, offsets, dictionary, None, cols[0].is_bool)
+
+
+def _concat_frames(frames: List[DeviceFrame]) -> DeviceFrame:
+    if not frames:
+        return DeviceFrame()
+    return DeviceFrame({name: _concat_columns([f[name] for f in frames]) for name in frames[0].columns})
 
 
 def _permute_rows(frame: DeviceFrame, perm: torch.Tensor) -> DeviceFrame:

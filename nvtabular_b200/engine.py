@@ -575,3 +575,126 @@ class GroupStats:
             _lib.ptr_array([o.data_ptr() for o in outs]), _lib.int_array(codes), _lib.stream_ptr()))
         _count()
         return outs
+
+
+# ------------------------------------------------------------------ session ops (csrc/groupby.cu)
+AGG_SLOTS = ("count", "sum", "mean", "min", "max", "std", "var", "first", "last")
+
+
+def _validity_buf(n: int, device) -> torch.Tensor:
+    """a zeroed bitmask for n rows, padded to 32 bytes like pack_validity"""
+    return torch.zeros(max((((n + 7) // 8 + 31) // 32) * 32, 32), dtype=torch.uint8, device=device)
+
+
+def sort_rows(keys: Sequence[Column], descending: Optional[Sequence[bool]] = None, n_drop_null: int = 0):
+    """stable row order by `keys` (first most significant), nulls of the first `n_drop_null` keys
+    dropped, other nulls last (nvtb_sort_rows) -> (perm int32[n], kept-row count as a device
+    int64[1]); the kept rows are perm[:n_kept]"""
+    _lib.require_cuda()
+    lib = _lib.load()
+    n = _check_same_len(keys)
+    dev = keys[0].data.device
+    perm = torch.empty(n, dtype=torch.int32, device=dev)
+    n_kept = torch.empty(1, dtype=torch.int64, device=dev)
+    desc = [1 if d else 0 for d in (descending or [False] * len(keys))]
+    with _timed("sort_rows", _in_bytes(keys) * 8):
+        _lib.check(lib.nvtb_sort_rows(_descs(keys), _lib.int_array(desc), len(keys), int(n_drop_null), n,
+                                      _ptr(perm), _ptr(n_kept), _lib.stream_ptr()))
+    _count(4 + 8 * len(keys))
+    return perm, n_kept
+
+
+def segments(keys: Sequence[Column], perm: torch.Tensor, n_kept: torch.Tensor):
+    """group boundaries of the sorted keys (nvtb_segments; synchronises) ->
+    (offsets int64[n_groups + 1], n_groups, kept rows)"""
+    lib = _lib.load()
+    n = perm.numel()
+    offsets = torch.empty(n + 1, dtype=torch.int64, device=perm.device)
+    ng, nk = c_int64(0), c_int64(0)
+    _lib.check(lib.nvtb_segments(_descs(keys), len(keys), _ptr(perm), n, _ptr(n_kept), _ptr(offsets),
+                                 byref(ng), byref(nk), _lib.stream_ptr()))
+    _count(4)
+    return offsets[: ng.value + 1], ng.value, nk.value
+
+
+def gather_rows(col: Column, perm: Optional[torch.Tensor], n: int, idx: Optional[torch.Tensor] = None,
+                shift: int = 0) -> Column:
+    """flat column rows col[perm[idx[i] + shift]] (nvtb_gather_rows); keeps the dictionary / bool flag"""
+    lib = _lib.load()
+    dev = col.data.device
+    out = torch.empty(n, dtype=col.data.dtype, device=dev)
+    valid = _validity_buf(n, dev) if col.validity is not None else None
+    _lib.check(lib.nvtb_gather_rows(_descs([col]), _ptr(perm), _ptr(idx), int(shift), n, _ptr(out), _ptr(valid),
+                                    _lib.stream_ptr()))
+    _count()
+    return Column(out, valid, None, col.dictionary, None, col.is_bool)
+
+
+def segment_agg(col: Column, perm: torch.Tensor, offsets: torch.Tensor, n_groups: int, aggs: Sequence[str]):
+    """{agg: Column} for aggs in AGG_SLOTS over every group (nvtb_segment_agg)"""
+    lib = _lib.load()
+    dev = col.data.device
+    outs, valids, res = [None] * 9, [None] * 9, {}
+    for a in aggs:
+        s = AGG_SLOTS.index(a)
+        dt = torch.int32 if a == "count" else torch.float32 if a in ("sum", "mean", "std", "var") else col.data.dtype
+        outs[s] = torch.empty(n_groups, dtype=dt, device=dev)
+        if a in ("mean", "min", "max", "std", "var") or (a in ("first", "last") and col.validity is not None):
+            valids[s] = _validity_buf(n_groups, dev)
+        keep_meta = a in ("min", "max", "first", "last")
+        res[a] = Column(outs[s], valids[s], None, col.dictionary if keep_meta else None, None,
+                        col.is_bool and keep_meta)
+    with _timed("segment_agg", _in_bytes([col]) + 4.0 * perm.numel()):
+        _lib.check(lib.nvtb_segment_agg(_descs([col]), _ptr(perm), _ptr(offsets), n_groups,
+                                        _lib.ptr_array([o.data_ptr() if o is not None and o.numel() else None
+                                                        for o in outs]),
+                                        _lib.ptr_array([v.data_ptr() if v is not None else None for v in valids]),
+                                        _lib.stream_ptr()))
+    _count(6)
+    return res
+
+
+def segment_sorted_agg(col: Column, perm: torch.Tensor, offsets: torch.Tensor, n_groups: int, n_rows: int,
+                       median=False, nunique=False):
+    """{"median": Column, "nunique": Column} over groups in value order (nvtb_segment_sorted_agg)"""
+    lib = _lib.load()
+    dev = col.data.device
+    res = {}
+    med = torch.empty(n_groups, dtype=torch.float32, device=dev) if median else None
+    med_v = _validity_buf(n_groups, dev) if median else None
+    nun = torch.empty(n_groups, dtype=torch.int32, device=dev) if nunique else None
+    _lib.check(lib.nvtb_segment_sorted_agg(_descs([col]), _ptr(perm), _ptr(offsets), n_groups, n_rows,
+                                           _ptr(med) if median else None, _ptr(med_v) if median else None,
+                                           _ptr(nun) if nunique else None, _lib.stream_ptr()))
+    _count(4)
+    if median:
+        res["median"] = Column(med, med_v)
+    if nunique:
+        res["nunique"] = Column(nun)
+    return res
+
+
+def list_slice(col: Column, start: int, end: int, pad: bool = False, max_elements: int = 0, pad_value: float = 0.0,
+               perm: Optional[torch.Tensor] = None, idx: Optional[torch.Tensor] = None, shift: int = 0,
+               n_rows: Optional[int] = None) -> Column:
+    """rows row[start:end] (Python slicing, padded to max_elements when `pad`) of a list column,
+    optionally through a row permutation (nvtb_list_slice_offsets + nvtb_list_slice)"""
+    _lib.require_cuda()
+    lib = _lib.load()
+    assert col.offsets is not None, "list_slice needs a list column"
+    dev = col.data.device
+    n = col.nrows if n_rows is None else n_rows
+    offsets = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    total = c_int64(0)
+    _lib.check(lib.nvtb_list_slice_offsets(_ptr(col.offsets), n, _ptr(perm), _ptr(idx), int(shift), int(start),
+                                           int(end), 1 if pad else 0, int(max_elements), _ptr(offsets), byref(total),
+                                           _lib.stream_ptr()))
+    t = total.value
+    leaves = torch.empty(t, dtype=col.data.dtype, device=dev)
+    valid = _validity_buf(t, dev) if col.validity is not None else None
+    with _timed("list_slice", 2.0 * t * col.data.element_size() + 16.0 * n):
+        _lib.check(lib.nvtb_list_slice(_ptr(col.offsets), _descs([col]), n, _ptr(perm), _ptr(idx), int(shift),
+                                       int(start), int(end), 1 if pad else 0, int(max_elements), float(pad_value),
+                                       _ptr(offsets), t, _ptr(leaves), _ptr(valid), _lib.stream_ptr()))
+    _count(4)
+    return Column(leaves, valid, offsets, col.dictionary, None, col.is_bool)

@@ -4,8 +4,10 @@ from .base import Operator, StatOperator  # noqa: F401
 from .categorify import Categorify  # noqa: F401
 from .clip_log import Clip, LogOp  # noqa: F401
 from .fill import FillMissing  # noqa: F401
+from .groupby import Groupby  # noqa: F401
 from .hash_bucket import HashBucket, emb_sz_rule  # noqa: F401
 from .join_groupby import JoinGroupby  # noqa: F401
+from .list_slice import ListSlice  # noqa: F401
 from .normalize import Normalize, NormalizeMinMax  # noqa: F401
 from .target_encoding import TargetEncoding  # noqa: F401
 

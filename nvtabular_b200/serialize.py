@@ -240,7 +240,17 @@ def _registry():
             lambda p, s, adir: ops.HashBucket(num_buckets=p["num_buckets"])),
         "nvtabular.ops.join_groupby.JoinGroupby": (ops.JoinGroupby, _join_groupby_to, _join_groupby_from),
         "nvtabular.ops.target_encoding.TargetEncoding": (ops.TargetEncoding, _target_encoding_to, _target_encoding_from),
+        # graph_serializer.py:450-471 of the reference
+        "nvtabular.ops.list_slice.ListSlice": (
+            ops.ListSlice, lambda op, adir: ({"start": op.start, "end": op.end, "pad": op.pad, "pad_value": op.pad_value}, {}),
+            lambda p, s, adir: ops.ListSlice(start=p["start"], end=p.get("end"), pad=p.get("pad", False),
+                                             pad_value=p.get("pad_value", 0.0))),
     }
+
+
+# operators the reference's serializer refuses (graph_serializer.py:919-929); refusing them too keeps
+# graph.json readable by either implementation
+_DEFERRED = {"Groupby"}
 
 
 _KIND_CLASS = {"input": "merlin.dag.ops.selection.SelectionOp", "concat": "merlin.dag.ops.concat_columns.ConcatColumns",
@@ -267,6 +277,10 @@ def save_workflow(workflow, path):
         i = ids[id(n)]
         adir = os.path.join(path, "artifacts", f"node_{i}")
         if n.kind == "op":
+            if type(n.op).__name__ in _DEFERRED:
+                raise NotImplementedError(
+                    f"The operator '{type(n.op).__name__}' is not yet supported by the JSON workflow "
+                    "serializer. Please open an issue or use a supported operator.")
             entry = by_cls.get(type(n.op))
             if entry is None:
                 raise WorkflowSerializationError(f"no serializer for operator {type(n.op).__name__}")

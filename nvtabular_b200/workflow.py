@@ -24,6 +24,20 @@ from .ops.base import Operator, StatOperator
 from .ops.fill import materialize_many
 
 
+def _merge_frames(node: Node, sources: List[Node], frames: List[DeviceFrame]) -> DeviceFrame:
+    """the columns of several upstream frames as one frame; they must have the same rows (a
+    Groupby upstream of only some of them changes the row count)"""
+    lens = {id(s): len(f) for s, f in zip(sources, frames) if f.columns}
+    if len(set(lens.values())) > 1:
+        detail = ", ".join(f"{s!r}: {lens[id(s)]} rows" for s in sources if id(s) in lens)
+        raise ValueError(f"{node!r} merges inputs with different row counts ({detail})")
+    out = DeviceFrame()
+    for f in frames:
+        for k, v in f.items():
+            out[k] = v
+    return out
+
+
 def _execute_node(node: Node, root: DeviceFrame, cache: Dict[int, DeviceFrame]) -> DeviceFrame:
     hit = cache.get(id(node))
     if hit is not None:
@@ -36,19 +50,13 @@ def _execute_node(node: Node, root: DeviceFrame, cache: Dict[int, DeviceFrame]) 
     else:
         frames = [_execute_node(p, root, cache) for p in node.upstream]
         if node.kind in ("concat",):
-            out = DeviceFrame()
-            for f in frames:
-                for k, v in f.items():
-                    out[k] = v
+            out = _merge_frames(node, node.upstream, frames)
         elif node.kind == "subtract":
             out = frames[0].drop(node.selector.names)
         elif node.kind == "subset":
             out = frames[0][node.selector.names]
         else:
-            inp = DeviceFrame()
-            for f in frames:
-                for k, v in f.items():
-                    inp[k] = v
+            inp = _merge_frames(node, node.upstream, frames)
             if not node.op.fuses_fill:
                 names = inp.columns
                 cols = materialize_many([inp[n] for n in names])
@@ -102,11 +110,8 @@ class _UpstreamPartitions:
     def __iter__(self):
         for part in self.dataset.partitions():
             cache: Dict[int, DeviceFrame] = {}
-            out = DeviceFrame()
-            for up in self.node.upstream:
-                for k, v in _execute_node(up, part, cache).items():
-                    out[k] = v
-            yield out
+            ups = self.node.upstream
+            yield _merge_frames(self.node, ups, [_execute_node(up, part, cache) for up in ups])
 
 
 class Workflow:
